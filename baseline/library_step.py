@@ -1,5 +1,5 @@
 """The "library Blackwell path to beat" (SURVEY 8d): the UNMODIFIED reference model / loss / step
-(baseline/_ref, see ref_loader.py) on device='cuda' -- torch's own kernels (cuBLASLt, cuDNN conv,
+(oracle/_ref, see ref_loader.py) on device='cuda' -- torch's own kernels (cuBLASLt, cuDNN conv,
 F.layer_norm, nn.GELU, nn.MultiheadAttention/SDPA, autograd, torch AdamW) under the flags of the
 reference's GPU scripts (scripts/exp/gpu/*: --precision amp_bf16 --grad-checkpointing --local-loss
 --gather-with-grad, TF32 + cudnn.benchmark as training/main.py:85-91).  A measurement, never on the
@@ -64,7 +64,7 @@ def library_baseline(wl: dict, batch: int, steps: int = 3, warmup: int = 2, grad
     e1.record()
     torch.cuda.synchronize(dev)
     ms = e0.elapsed_time(e1) / steps
-    out = {"path": "unmodified reference (baseline/_ref) on torch CUDA library kernels, amp_bf16"
+    out = {"path": "unmodified reference (oracle/_ref) on torch CUDA library kernels, amp_bf16"
                    + (", grad checkpointing" if grad_checkpointing else ""),
            "model": wl["model"], "image_px": wl["image"], "batch": batch, "steps": steps, "warmup": warmup,
            "ms_per_step": ms, "pairs_per_s": batch / (ms * 1e-3), "loss": float(loss),

@@ -1,9 +1,8 @@
 """Imports the UNMODIFIED reference (`open_clip` + `training` of UCSC-VLAA/CLIPA clipa_torch) for
 measurement and drop-in tests.  Never imported by the product path (clipa_b200/).
 
-Where it comes from: `baseline/_ref/` -- `python -m pip install --no-index --no-build-isolation --no-deps
---target baseline/_ref <copy of /root/reference/clipa_torch>` (tools/install_reference.sh; git-ignored,
-travels to the GPU box) -- or, in the authoring container only, /root/reference/clipa_torch itself.
+Where it comes from: `oracle/_ref/`, filled from a clipa_torch checkout by `oracle/install_reference.sh`
+(git-ignored).  Nothing else is searched: tests compare against the committed vectors under tests/golden.
 
 The reference's tokenizer / data modules import ftfy, tensorflow(_text), webdataset, braceexpand
 unconditionally (open_clip/tokenizer.py:11-18, training/data.py:9,17-22); none of them is on the
@@ -21,16 +20,13 @@ from pathlib import Path
 from unittest.mock import MagicMock
 
 ROOT = Path(__file__).resolve().parent.parent
-CANDIDATES = (ROOT / "baseline" / "_ref", Path("/root/reference/clipa_torch"))
+REF_DIR = ROOT / "oracle" / "_ref"
 _STUBS = ("ftfy", "tensorflow", "tensorflow_text", "webdataset", "webdataset.filters",
           "webdataset.tariterators", "braceexpand", "fsspec", "timm", "horovod", "horovod.torch")
 
 
 def reference_root():
-    for c in CANDIDATES:
-        if (c / "open_clip" / "factory.py").exists():
-            return c
-    return None
+    return REF_DIR if (REF_DIR / "open_clip" / "factory.py").exists() else None
 
 
 def available() -> bool:
@@ -41,7 +37,7 @@ def import_reference(register_configs: bool = True):
     """Returns the reference's `open_clip` module (its `training` package becomes importable too)."""
     root = reference_root()
     if root is None:
-        raise RuntimeError("reference not installed: run tools/install_reference.sh in the authoring container")
+        raise RuntimeError(f"reference not installed in {REF_DIR}: run oracle/install_reference.sh <clipa_torch dir>")
     for n in _STUBS:
         if n not in sys.modules:
             try:

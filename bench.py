@@ -175,15 +175,38 @@ def cpu_baseline(wl, budget_s=20.0, batch=8):
                       f"batch {batch}, {n} steps after 1 warm-up, fp32, torch CPU threads={cores}"}
 
 
+DUMP_SAMPLE = 1 << 22     # parameter elements written by --dump-outputs (16 MB of float32)
+
+
+def dump_outputs(out_dir: Path, loss, model) -> None:
+    """What a caller of the timed step holds after its last step, as float32 .npy files: the loss it returned and the
+    parameters it updated (logit_scale whole; the rest as a fixed, seeded sample of DUMP_SAMPLE elements of all
+    parameters concatenated in named_parameters() order, in ascending position)."""
+    import numpy as np
+    import torch
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "loss.npy", np.asarray([float(loss)], dtype=np.float32))
+    np.save(out_dir / "logit_scale.npy", model.logit_scale.detach().float().reshape(1).cpu().numpy())
+    flat = [p.detach().reshape(-1) for _, p in model.named_parameters()]
+    sizes = torch.tensor([t.numel() for t in flat])
+    ends = torch.cumsum(sizes, 0)
+    total = int(ends[-1])
+    idx, _ = torch.sort(torch.randint(0, total, (min(DUMP_SAMPLE, total),), generator=torch.Generator().manual_seed(0)))
+    lo, hi = torch.searchsorted(idx, ends - sizes).tolist(), torch.searchsorted(idx, ends).tolist()
+    vals = torch.cat([t[(idx[a:b] - int(e - n)).to(t.device)].float().cpu()
+                      for t, a, b, e, n in zip(flat, lo, hi, ends.tolist(), sizes.tolist())])
+    np.save(out_dir / "params_sample.npy", vals.numpy())
+
+
 def library_baseline_leg(wl, batch):
     """Bounded sample of the "library Blackwell path to beat" (SURVEY 8d): the unmodified reference
-    (baseline/_ref) on torch's CUDA kernels, same box, right after our timed region.  Reported beside the
+    (oracle/_ref) on torch's CUDA kernels, same box, right after our timed region.  Reported beside the
     headline, never part of it."""
     import gc
     import torch
     from baseline.ref_loader import available
     if not available():
-        return {"unavailable": "baseline/_ref not installed (tools/install_reference.sh)"}
+        return {"unavailable": "oracle/_ref not installed (oracle/install_reference.sh)"}
     gc.collect()
     torch.cuda.empty_cache()
     torch.cuda.reset_peak_memory_stats()
@@ -247,6 +270,9 @@ def main():
     ap.add_argument("--save-ln", default="auto", choices=["auto", "on", "off"],
                     help="keep LayerNorm outputs for backward (auto: when HBM allows)")
     ap.add_argument("--op-table", default=None, help="write the per-kernel CUDA-event table (JSON) to this path")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the last step's loss and updated parameters (a fixed sample) "
+                         "to DIR/*.npy, to compare two builds output for output")
     args = ap.parse_args()
     name = args.workload
     wl = dict(WORKLOADS[name])
@@ -331,6 +357,8 @@ def main():
 
     # ---- device-resident throughput (`value`): uninstrumented region ----
     ms_step, launches, clocks, _, last_loss = timed(lambda: trainer.step(d_images, d_text), args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), last_loss, model)
     value = gb / (ms_step * 1e-3)
     # ---- second pass with the per-launch CUDA-event profiler on: roofline of the GEMM kernels + op table ----
     prof_steps = max(1, args.steps // 2)

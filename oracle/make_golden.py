@@ -1,8 +1,7 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (imported from
-/root/reference/clipa_torch) on seeded synthetic weights and inputs.
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (imported from oracle/_ref, installed by
+oracle/install_reference.sh) on seeded synthetic weights and inputs, on the CPU.
 
-Runs only in the authoring container (the GPU box has no /root/reference); the vectors it writes are
-committed.  Usage:  python oracle/make_golden.py
+The vectors it writes are committed; the tests read only those.  Usage:  python oracle/make_golden.py
 
 What is pinned per case (fp32 reference run, plus a pure-bf16 run that calibrates the bf16
 tolerance): image/text features, loss, and gradients of logit_scale, visual.proj, text_projection,
@@ -27,7 +26,7 @@ sys.path.insert(0, str(ROOT))
 from oracle.weights import (BASELINE_DIM_BATCH, BASELINE_DIM_CASES, CONFIG1, TINY_CONFIGS, make_inputs,  # noqa: E402
                             make_state_dict)
 
-REF = "/root/reference/clipa_torch"
+REF = str(ROOT / "oracle" / "_ref")
 GOLD = ROOT / "tests" / "golden"
 
 
